@@ -1,4 +1,4 @@
-"""Run the UNMODIFIED reference (siboehm/ShallowSpeed, installed in baseline/_ref) through
+"""Run the UNMODIFIED reference (siboehm/ShallowSpeed, installed in oracle/_ref by build()) through
 its own public API - the same objects and loop as its train.py:98-146 (MLP, SGD, Dataset,
 Worker, schedules) - on MNIST-shaped synthetic data, and time K training steps.
 
@@ -17,10 +17,11 @@ import time
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
+REF = HERE.parent / "oracle" / "_ref"
 
 
 def reference_available():
-    return (HERE / "_ref" / "shallowspeed" / "pipe.py").exists()
+    return (REF / "shallowspeed" / "pipe.py").exists()
 
 
 def main(argv=None):
@@ -44,7 +45,7 @@ def main(argv=None):
     for v in ("OMP_NUM_THREADS", "OPENBLAS_NUM_THREADS", "MKL_NUM_THREADS"):
         os.environ[v] = str(threads)          # upper bound of the BLAS pool; the sweep below lowers it at run time
     sys.path.insert(0, str(HERE / "mpi_shim"))
-    sys.path.insert(0, str(HERE / "_ref"))
+    sys.path.insert(0, str(REF))
     import numpy as np
     from mpi4py import MPI
     from shallowspeed.dataset import Dataset

@@ -14,6 +14,8 @@ default workload - MLP 784-128-127-126-125-124-123-10, 4 micro-batches, SGD lr 0
                global batch = 128 x N.  ``--scaling strong`` keeps the global batch at 128.
 * ``--impl reference`` runs the unmodified reference (NumPy on the host CPUs, mpi4py shim)
                on the same config; N ranks = N processes.
+* ``--dump-outputs DIR`` writes the loss and the parameters of the last timed step as .npy files, so that two
+               builds run with the same arguments (same seeded inputs and initial weights) can be compared.
 """
 from __future__ import annotations
 
@@ -55,7 +57,12 @@ def parse():
     ap.add_argument("--repeats", type=int, default=5, help="the K-step block is timed this many times; the MEDIAN block is reported")
     ap.add_argument("--no-exposed", action="store_true", help="skip the compute-only twin run that yields comm.exposed_ms_per_step")
     ap.add_argument("--ref-threads", type=int, default=0, help="reference arm: BLAS threads per rank (0 = calibrate over a sweep)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss of the last step and the parameters it left as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def relaunch_under_torchrun(args):
@@ -87,7 +94,7 @@ def run_reference(args):
     import run_reference as rr
 
     if not rr.reference_available():
-        print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref not installed (pip --target baseline/_ref /root/reference)"}))
+        print(json.dumps({"impl": "reference", "unavailable": "the original project is not installed in oracle/_ref (build() installs it from a checkout: oracle/install_reference.py)"}))
         return
     rank = int(os.environ.get("RANK", "0"))
     gbs = global_batch(args)
@@ -131,6 +138,40 @@ def run_reference(args):
                        "weights_dtype": res["weights_dtype"],
                        "timing": "wall clock between barriers, max over ranks (CPU code)"},
         }))
+
+
+DUMP_BUDGET = 15_000_000   # float32 values (60 MB): the dump stays under 64 MB with the biases and the loss
+
+
+def dump_outputs(out_dir, trainer, grid, sizes, loss):
+    """What a caller of the timed path holds after its last step, as float32 ``.npy`` files: ``loss`` (shape (1,),
+    from the last pipeline stage) and, per layer (global index ``i``), ``W<i>`` (out, in) and ``b<i>`` (out,).
+    DP replica 0 writes; each pipeline stage writes its own layers.  When all parameters together exceed
+    ``DUMP_BUDGET`` values, every weight matrix is written as ``W<i>_sample``: the elements at a fixed set of flat
+    indices drawn from a RandomState seeded with ``i``, so two runs with the same arguments sample the same elements."""
+    import numpy as np
+    import torch
+
+    from shallowspeed_b200.models.mlp import stage_layer_specs
+
+    if grid.replica != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    trainer.synchronize()
+    arena = trainer.model.arena
+    total = sum(i * o + o for i, o in zip(sizes[:-1], sizes[1:]))
+    frac = min(1.0, DUMP_BUDGET / total)
+    for bi, (n_in, n_out, _relu, layer) in enumerate(stage_layer_specs(sizes, grid.stage, grid.pp)):
+        w = arena.weight_view(bi)
+        if frac < 1.0:
+            rs = np.random.RandomState(layer)
+            flat = torch.from_numpy(np.sort(rs.randint(0, n_out * n_in, int(frac * n_out * n_in)))).to(w.device)
+            np.save(os.path.join(out_dir, f"W{layer}_sample.npy"), w[flat // n_in, flat % n_in].float().cpu().numpy())
+        else:
+            np.save(os.path.join(out_dir, f"W{layer}.npy"), w.float().cpu().numpy())
+        np.save(os.path.join(out_dir, f"b{layer}.npy"), arena.bias_view(bi).reshape(-1).float().cpu().numpy())
+    if loss is not None:
+        np.save(os.path.join(out_dir, "loss.npy"), np.array([loss], dtype=np.float32))
 
 
 # ----------------------------------------------------------------------------------------
@@ -237,6 +278,8 @@ def run_ours(args):
         e2e_samples = timed_blocks(e2e_step, args.steps, args.repeats, stream)
         losses.append(trainer.flush())
     sampler[0] = None
+    if args.dump_outputs:   # now, while the trainer's last step is the last timed e2e step (SSB_COMM_TIMING runs one more)
+        dump_outputs(args.dump_outputs, trainer, grid, sizes, losses[-1])
     ms_dev, dev_blocks = reduce_blocks(dev_samples)
     ms_e2e, e2e_blocks = reduce_blocks(e2e_samples)
     clocks = clk.summary()

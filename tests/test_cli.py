@@ -57,8 +57,8 @@ def test_train_rejects_bad_grids():
     assert r.returncode != 0            # 128 % 3 != 0 / world size mismatch
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "baseline", "_ref", "shallowspeed", "pipe.py")),
-                    reason="reference not installed in baseline/_ref")
+@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "shallowspeed", "pipe.py")),
+                    reason="original project not installed in oracle/_ref (build() installs it from a checkout)")
 def test_bench_reference_arm_json_contract():
     r = _run(["bench.py", "--impl", "reference", "--steps", "5", "--warmup", "3"])
     assert r.returncode == 0, r.stderr[-2000:]
@@ -68,6 +68,74 @@ def test_bench_reference_arm_json_contract():
         assert key in d, key
     assert d["impl"] == "reference" and d["n_gpus"] == 1 and d["steps"] == 5 and d["value"] > 0
     assert d["config"]["global_batch"] == 128 and d["config"]["n_mubatches"] == 4
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("model,budget", [([], None), (["--hidden", "256", "--n-layers", "4"], 50_000)])
+def test_bench_dump_outputs(model, budget, tmp_path, monkeypatch, capsys):
+    """bench.py --dump-outputs, run in this process so the trainer can be watched: the trainer takes exactly the
+    warm-up and timed steps --warmup / --steps / --repeats ask for, and the files hold its loss and parameters after
+    the last of them - in full, or (over the size budget) at the documented seeded sample of each weight matrix."""
+    import numpy as np
+
+    sys.path.insert(0, ROOT)
+    try:
+        import bench
+    finally:
+        sys.path.remove(ROOT)
+    from shallowspeed_b200.layers import MLP
+    from shallowspeed_b200.parallel.engine import Trainer
+
+    trainers = {}
+    step_async = Trainer.step_async
+
+    def counting_step_async(self, x, y):
+        trainers[self] = trainers.get(self, 0) + 1
+        return step_async(self, x, y)
+
+    monkeypatch.setattr(Trainer, "step_async", counting_step_async)
+    monkeypatch.delenv("SSB_COMM_TIMING", raising=False)
+    if budget:
+        monkeypatch.setattr(bench, "DUMP_BUDGET", budget)
+    out = tmp_path / "dump"
+    steps, warmup, repeats = 3, 5, 2
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", str(steps), "--warmup", str(warmup), "--repeats", str(repeats),
+                                      "--no-alt", "--pool-batches", "8", "--dump-outputs", str(out)] + model)
+    args = bench.parse()
+    bench.run_ours(args)
+    d = json.loads([l for l in capsys.readouterr().out.splitlines() if l.startswith("{")][-1])
+    (trainer, n_steps), = trainers.items()
+    # device-timed arm, then the e2e arm: warm-up, then `repeats` blocks of one aligning + `steps` timed steps each
+    assert n_steps == max(3, warmup) + max(3, warmup // 4) + 2 * repeats * (steps + 1)
+    assert d["steps"] == steps and len(d["timing"]["block_ms"]) == len(d["e2e"]["block_ms"]) == repeats
+
+    sizes = bench.layer_sizes(args)
+    total = sum(i * o + o for i, o in zip(sizes[:-1], sizes[1:]))
+    frac = min(1.0, bench.DUMP_BUDGET / total)
+    names, nbytes = [], 0
+    init = MLP(sizes, 0, 1, 128).parameters()
+    arena = trainer.model.arena
+    for i, (n_in, n_out) in enumerate(zip(sizes[:-1], sizes[1:])):
+        w_now = arena.weight_view(i).cpu().numpy()
+        if frac < 1.0:
+            names.append(f"W{i}_sample.npy")
+            w = np.load(out / names[-1])
+            idx = np.sort(np.random.RandomState(i).randint(0, n_out * n_in, int(frac * n_out * n_in)))
+            assert w.shape == idx.shape and np.array_equal(w, w_now.reshape(-1)[idx])
+        else:
+            names.append(f"W{i}.npy")
+            w = np.load(out / names[-1])
+            assert w.shape == (n_out, n_in) and np.array_equal(w, w_now)
+            assert not np.array_equal(w, init[2 * i].data.numpy())      # trained, not the initial weights
+        names.append(f"b{i}.npy")
+        b = np.load(out / names[-1])
+        assert b.shape == (n_out,) and np.array_equal(b, arena.bias_view(i).reshape(-1).cpu().numpy())
+        assert w.dtype == b.dtype == np.float32 and np.isfinite(w).all()
+        nbytes += w.nbytes + b.nbytes
+    loss = np.load(out / "loss.npy")
+    assert loss.dtype == np.float32 and loss.shape == (1,) and loss[0] == np.float32(trainer.loss()) == np.float32(d["config"]["last_loss"])
+    assert sorted(p.name for p in out.iterdir()) == sorted(names + ["loss.npy"])
+    assert nbytes <= 4 * (bench.DUMP_BUDGET + sum(sizes[1:]))
 
 
 def test_blocking_ddp_contrast_script(tmp_path):

@@ -94,15 +94,20 @@ def test_watchdog_reports_and_aborts_on_timeout(monkeypatch):
     assert w._pp_nccl.aborted
 
 
-def test_fd_passing_over_unix_socket(tmp_path):
+def test_fd_passing_over_unix_socket(request):
     """NVLS set-up hands the multicast object's POSIX fd to the other replicas with SCM_RIGHTS; check the transport
     with a pipe: what the peers write into the received descriptors arrives at the leader's read end."""
     import os
+    import shutil
+    import tempfile
 
     from shallowspeed_b200.parallel import engine as E
 
+    # AF_UNIX socket paths are limited to 107 bytes, which pytest's tmp_path under a deep $TMPDIR can exceed
+    sock_dir = tempfile.mkdtemp(prefix="ssb_fd_", dir="/tmp")
+    request.addfinalizer(lambda: shutil.rmtree(sock_dir, ignore_errors=True))
     r, w = os.pipe()
-    path = str(tmp_path / "fd.sock")
+    path = os.path.join(sock_dir, "fd.sock")
     srv = E.serve_fd(path, w, 2)
     got = []
 
